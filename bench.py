@@ -6,6 +6,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...      # the reference's own CPU path on the host cores
+    python bench.py --gpus 1 --steps 200 --warmup 20 --dump-outputs DIR   # + what the last timed step computed
 
 One "step" = one env-step of every environment (PD -> ABA -> integrate -> collide -> LCP/PGS ->
 integrate).  Environments are sharded across ranks (4096 per GPU: weak scaling), there is no
@@ -20,6 +21,10 @@ import threading
 import time
 
 import numpy as np
+
+# the benchmark writes nothing into the tree it runs from, writable or not: without this, the first import of a module
+# (tds_b200.parallel, oracle.ref, ...) leaves a __pycache__ directory beside its source
+sys.dont_write_bytecode = True
 
 # stdout carries exactly ONE JSON line: everything else that libraries print there (NCCL's version banner, the
 # reference's "Loading URDF" chatter) is sent to stderr by pointing fd 1 at fd 2; the result goes to the saved fd.
@@ -38,6 +43,27 @@ ENVS_PER_GPU = 4096
 ALGO_BYTES_PER_ENV_STEP = 344       # SURVEY.md section 8d: q18+qd18+action12 read, q18+qd18+reward+done written (fp32)
 FLOPS_PER_ENV_STEP = 27e3           # op count of the reference's CppAD tape (SURVEY.md section 8d)
 METRIC = "env-steps/sec (N parallel sims)"
+DUMP_LIMIT_BYTES = 64_000_000
+
+
+def dump_outputs(dirname, arrays):
+    """--dump-outputs: writes each array (one row per environment) as <dirname>/<name>.npy, float32 or float64 (integer
+    outputs as float64), so that two builds run with the same arguments can be compared output for output.  Above
+    DUMP_LIMIT_BYTES in all, the same fixed, seeded sample of environments is kept from every array; env_index.npy then
+    lists which."""
+    arrays = {k: np.asarray(v) for k, v in arrays.items()}
+    arrays = {k: v if v.dtype in (np.float32, np.float64) else v.astype(np.float64) for k, v in arrays.items()}
+    n = next(iter(arrays.values())).shape[0]
+    row_bytes = sum(v.nbytes for v in arrays.values()) // n
+    budget = DUMP_LIMIT_BYTES - 4096 * (len(arrays) + 1)   # room for the .npy headers
+    if n * row_bytes > budget:
+        keep = budget // (row_bytes + 8)
+        idx = np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+        arrays = {k: v[idx] for k, v in arrays.items()}
+        arrays["env_index"] = idx.astype(np.float64)
+    os.makedirs(dirname, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(dirname, k + ".npy"), np.ascontiguousarray(v))
 
 
 def _measured_peaks():
@@ -394,6 +420,14 @@ def run_config(args, rank, world, local_rank):
     total_ms = float(t.item())
     if not bool(torch.isfinite(q2).all()) or not bool(torch.isfinite(qd2).all()):
         raise SystemExit("bench.py: non-finite state after the timed region")
+    if args.dump_outputs and rank == 0:   # what step_device / the contact record of the last timed step returned
+        def rows(t, dim):
+            return t[:dim, :n].T.cpu().numpy()
+        out = {"qdd": rows(qdd, sim.n_qd)} if mode == 0 else {"q": rows(q2, sim.n_q), "qd": rows(qd2, sim.n_qd)}
+        if cdist is not None:
+            out.update(contact_dist=rows(cdist, sim.n_contact_points), contact_count=ccount[:n].cpu().numpy(),
+                       contact_links=rows(clinks, 2 * sim.n_contact_points))
+        dump_outputs(args.dump_outputs, out)
     # end to end through tds_b200_step_host: fp64 AoS host buffers in and out (the MultiBody-style arrays a
     # VectorizedEnvironment caller holds), copies + layout conversion + step inside the timed region
     hq, hqd = w["q"].copy(), w["qd"].copy()
@@ -461,7 +495,12 @@ def main():
                          "writes into the NCCL send buffer, the collective is captured in the same CUDA graph")
     ap.add_argument("--gather-overlap", action="store_true", help="with --gather-reward: the gather of step k runs on a side stream under step k+1")
     ap.add_argument("--strong", action="store_true", help="strong scaling: the config's environments are divided over the ranks")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned (rank 0's environments) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        # the reference arms size their batch from a measured rate, so their outputs differ from run to run
+        ap.error("--dump-outputs needs --impl b200")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -556,6 +595,17 @@ def main():
     if sampler:
         sampler.start()
         time.sleep(0.25)
+
+    def last_outputs():
+        """What the env step returned in the last timed step (one_step(W + K)): the resident state the observations are
+        read from, reward and done.  Called after the closing event, so it is not timed."""
+        if not args.dump_outputs or rank != 0:
+            return None
+        torch.cuda.synchronize()
+        q_o, qd_o = sim.env_get_state()
+        r, d = (reward, done) if gathered is None else (gathered.reward(W + K), gathered.done(W + K))
+        return {"q": q_o, "qd": qd_o, "reward": r[:n].cpu().numpy(), "done": d[:n].cpu().numpy()}
+
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     t_wall0 = time.perf_counter()
     reps = 1
@@ -570,6 +620,7 @@ def main():
         ev0.record()
         graph.replay()
         ev1.record()
+        outputs = last_outputs()
         for _ in range(reps - reps // 2 - 1):
             graph.replay()
         torch.cuda.synchronize()
@@ -580,6 +631,7 @@ def main():
         if gathered is not None:
             gathered.join()
         ev1.record()
+        outputs = last_outputs()
     torch.cuda.synchronize()
     if world > 1:
         dist.barrier()
@@ -594,6 +646,8 @@ def main():
     q_chk, _ = sim.env_get_state()
     if not np.all(np.isfinite(q_chk)):
         raise SystemExit("bench.py: non-finite state after the timed region")
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
 
     # ---- end-to-end through the public host API: pinned host actions in, obs/reward/done out, every step
     act_h = torch.rand((n, 12)).mul_(0.8).sub_(0.4).pin_memory()
