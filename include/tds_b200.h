@@ -123,6 +123,21 @@ int tds_b200_step_jacobian_device(tds_b200_sim* sim, int mode, int use_pd, const
 int tds_b200_step_jacobian_host(tds_b200_sim* sim, int mode, int use_pd, const double* q, const double* qd,
                                 const double* tau_or_action, double* jac);
 
+/* Jacobian-vector (forward mode) and vector-Jacobian (reverse mode: what a gradient needs) products of one step, without the
+ * dense Jacobian.  Same instance, rows (q' | qd', or qdd in mode FD) and input blocks (q | qd | tau, or action with use_pd;
+ * the PD-gain columns only through the dense Jacobian) as tds_b200_step_jacobian_device; q, qd, tau_or_action as in
+ * tds_b200_step_device (tau_or_action required with use_pd and whenever its tangent / gradient is).  Every tangent and
+ * gradient is fp64 [dim][n_stride]; padding columns (environment >= n) are not written.
+ *   jvp: t_q, t_qd, t_tau tangents of the input blocks (NULL = zero) -> t_out [rows][n_stride].  One dual lane per environment.
+ *   vjp: g_out cotangent [rows][n_stride] -> g_q, g_qd, g_tau (gradient of each block; NULL = not wanted, its directions are not
+ *        launched).  One dual lane per environment and wanted input direction; each writes one double.
+ * Return 0, -1 on a bad argument, -2 for TDS_B200_MODE_WORLD, -3 for use_pd without tds_b200_set_env, else a CUDA error.
+ * The scratch arena of the dual instance is shared with the dense Jacobian and only grows. */
+int tds_b200_step_jvp_device(tds_b200_sim* sim, int mode, int use_pd, const float* q, const float* qd, const float* tau_or_action,
+                             const double* t_q, const double* t_qd, const double* t_tau, double* t_out, void* stream);
+int tds_b200_step_vjp_device(tds_b200_sim* sim, int mode, int use_pd, const float* q, const float* qd, const float* tau_or_action,
+                             const double* g_out, double* g_q, double* g_qd, double* g_tau, void* stream);
+
 /* Stand-alone integration stages of the fine-grained surface (device SoA arrays as above):
  * integrate_euler (src/dynamics/integrator.hpp:10-133): qd += qdd dt (qdd may be NULL = zero), q += qd dt, floating base
  * quaternion increment + normalisation; integrate_euler_qdd (:141-195): qd += qdd dt only. */
@@ -292,6 +307,16 @@ int tds_b200_rigid_set_params(tds_b200_rigid* h, double dt, const double* gravit
 int tds_b200_rigid_step_device(tds_b200_rigid* h, const double* state_in, double* state_out, const double* force, int steps, void* stream);
 int tds_b200_rigid_step_host(tds_b200_rigid* h, const double* state, const double* force, int steps, double* state_out);
 int tds_b200_rigid_jacobian_host(tds_b200_rigid* h, const double* state, const double* force, int steps, double* state_out, double* jac);
+/* Jacobian-vector / vector-Jacobian products of `steps` steps with respect to (state | force), device layouts as
+ * tds_b200_rigid_step_device, tangents and gradients fp64 [13 * n_bodies][n_stride] (state) / [3 * n_bodies][n_stride] (force).
+ * One dual lane carries its derivative through all the steps, so memory does not grow with `steps`.  NULL force: zero force.
+ *   jvp: t_state, t_force (NULL = zero) -> t_out, one lane per world.
+ *   vjp: g_out -> g_state, g_force (NULL = not wanted, not launched), one lane per world and wanted input direction.
+ * stream NULL: the world's own stream. */
+int tds_b200_rigid_jvp_device(tds_b200_rigid* h, const double* state, const double* force, int steps,
+                              const double* t_state, const double* t_force, double* t_out, void* stream);
+int tds_b200_rigid_vjp_device(tds_b200_rigid* h, const double* state, const double* force, int steps,
+                              const double* g_out, double* g_state, double* g_force, void* stream);
 
 #ifdef __cplusplus
 }

@@ -12,3 +12,10 @@ from . import rigid  # noqa: F401
 from .sim import BatchSim, MODE_FD, MODE_NOCONTACT, MODE_FULL, MODE_WORLD, PREC_MIXED, PREC_F64, PREC_F32, PREC_AUTO  # noqa: F401
 from .envs import (VectorizedLaikagoEnv, VectorizedLaikagoEnvOutput, VectorizedAntEnv, CudaModelV1, laikago_sim,  # noqa: F401
                    ant_sim)
+
+
+def __getattr__(name):   # tds_b200.autograd (torch.autograd through the steps) imports torch: loaded on first use
+    if name == "autograd":
+        import importlib
+        return importlib.import_module(__name__ + ".autograd")
+    raise AttributeError(f"module {__name__!r} has no attribute {name!r}")

@@ -84,6 +84,10 @@ def lib():
     L.tds_b200_step_jacobian_device.argtypes = [vp, ci, ci, fp, fp, fp, vp, vp]
     L.tds_b200_step_jacobian_host.restype = ci
     L.tds_b200_step_jacobian_host.argtypes = [vp, ci, ci, dp, dp, dp, dp]
+    L.tds_b200_step_jvp_device.restype = ci
+    L.tds_b200_step_jvp_device.argtypes = [vp, ci, ci, fp, fp, fp, vp, vp, vp, vp, vp]
+    L.tds_b200_step_vjp_device.restype = ci
+    L.tds_b200_step_vjp_device.argtypes = [vp, ci, ci, fp, fp, fp, vp, vp, vp, vp, vp]
     L.tds_b200_integrate_euler_device.restype = ci
     L.tds_b200_integrate_euler_device.argtypes = [vp, fp, fp, fp, vp]
     L.tds_b200_integrate_euler_qdd_device.restype = ci
@@ -108,6 +112,10 @@ def lib():
     L.tds_b200_rigid_step_host.argtypes = [vp, vp, vp, ci, vp]
     L.tds_b200_rigid_jacobian_host.restype = ci
     L.tds_b200_rigid_jacobian_host.argtypes = [vp, vp, vp, ci, vp, vp]
+    L.tds_b200_rigid_jvp_device.restype = ci
+    L.tds_b200_rigid_jvp_device.argtypes = [vp, vp, vp, ci, vp, vp, vp, vp]
+    L.tds_b200_rigid_vjp_device.restype = ci
+    L.tds_b200_rigid_vjp_device.argtypes = [vp, vp, vp, ci, vp, vp, vp, vp]
     L.tds_b200_contact_tuples.restype = ci
     L.tds_b200_contact_tuples.argtypes = [vp, vp, ci]
     L.tds_b200_model_contact_tuples.restype = ci
@@ -151,8 +159,8 @@ DECLARED_SYMBOLS = [
     "b200_laikago_forward_zero_deallocate", "b200_laikago_forward_zero_send_local", "b200_laikago_forward_zero_send_global",
     "b200_laikago_jacobian", "b200_laikago_jacobian_meta", "b200_laikago_jacobian_allocate", "b200_laikago_jacobian_deallocate",
     "b200_laikago_jacobian_send_local", "b200_laikago_jacobian_send_global",
-    "tds_b200_jacobian_dims", "tds_b200_step_jacobian_device", "tds_b200_step_jacobian_host", "tds_b200_integrate_euler_device", "tds_b200_integrate_euler_qdd_device", "tds_b200_contact_pairs", "tds_b200_model_contact_pairs", "tds_b200_contact_tuples", "tds_b200_model_contact_tuples", "tds_b200_contact_list_device", "tds_b200_contact_list_host", "tds_b200_contact_list_candidates_host",
-    "tds_b200_rigid_create", "tds_b200_rigid_destroy", "tds_b200_rigid_set_params", "tds_b200_rigid_step_device", "tds_b200_rigid_step_host", "tds_b200_rigid_jacobian_host",
+    "tds_b200_jacobian_dims", "tds_b200_step_jacobian_device", "tds_b200_step_jacobian_host", "tds_b200_step_jvp_device", "tds_b200_step_vjp_device", "tds_b200_integrate_euler_device", "tds_b200_integrate_euler_qdd_device", "tds_b200_contact_pairs", "tds_b200_model_contact_pairs", "tds_b200_contact_tuples", "tds_b200_model_contact_tuples", "tds_b200_contact_list_device", "tds_b200_contact_list_host", "tds_b200_contact_list_candidates_host",
+    "tds_b200_rigid_create", "tds_b200_rigid_destroy", "tds_b200_rigid_set_params", "tds_b200_rigid_step_device", "tds_b200_rigid_step_host", "tds_b200_rigid_jacobian_host", "tds_b200_rigid_jvp_device", "tds_b200_rigid_vjp_device",
     "tds_b200_step_device", "tds_b200_step_host", "tds_b200_env_set_state_host",
     "tds_b200_env_get_state_host", "tds_b200_env_step_host", "tds_b200_env_step_device",
     "tds_b200_stream", "tds_b200_env_q", "tds_b200_env_qd", "cuda_model_laikago_forward_zero",

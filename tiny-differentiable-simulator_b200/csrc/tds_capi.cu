@@ -28,8 +28,8 @@ extern "C" size_t tds_spec_smem_bytes(int spec, int precision);
 extern "C" const char* tds_spec_name(int spec);
 extern "C" int tds_launch_step_spec(int spec, const SimParams* P, const EnvParams* E, const StepIO* io, int mode, int use_pd,
                                     int precision, cudaStream_t stream);
-extern "C" int tds_launch_stepw_jacobian(const DevModel* M, const SimParams* P, const EnvParams* E, const StepIO* io, int mode,
-                                         int use_pd, int n_dirs, char* gscratch, cudaStream_t stream);
+extern "C" int tds_launch_stepw_dual(const DevModel* M, const SimParams* P, const EnvParams* E, const StepIO* io, const DualIO* dio,
+                                     int mode, int use_pd, int n_dirs, char* gscratch, cudaStream_t stream);
 extern "C" int tds_launch_stepw(const DevModel* M, const SimParams* P, const EnvParams* E, const StepIO* io,
                                 int mode, int use_pd, int precision, char* gscratch, int use_smem,
                                 int warps_per_block, cudaStream_t stream);
@@ -763,6 +763,25 @@ int tds_b200_jacobian_dims(const tds_b200_sim* s, int mode, int use_pd, int dims
   return 0;
 }
 
+// Scratch of the dual-number instance for launches of up to `dirs` directions, bounded by 2 GB (more directions: several
+// launches of *chunk).  Grows only when a call needs more than the arena holds.
+static int ensure_dual_scratch(tds_b200_sim* s, int dirs, int* chunk) {
+  const size_t warps = (size_t)(s->n + 31) / 32;
+  const size_t per_dir = warps * (size_t)s->dm_ad.x_total * 32 * 4;
+  const size_t cap = (size_t)2 << 30;
+  int c = (int)(cap / per_dir);
+  if (c < 1) c = 1;
+  if (c > dirs) c = dirs;
+  if (per_dir * c > s->jac_scratch_bytes) {
+    if (s->jac_scratch) cudaFree(s->jac_scratch);
+    s->jac_scratch = nullptr; s->jac_scratch_bytes = 0;
+    CUDA_TRY(cudaMalloc((void**)&s->jac_scratch, per_dir * c));
+    s->jac_scratch_bytes = per_dir * c;
+  }
+  *chunk = c;
+  return 0;
+}
+
 int tds_b200_step_jacobian_device(tds_b200_sim* s, int mode, int use_pd, const float* q, const float* qd, const float* tau_or_action,
                                   double* jac, void* stream) {
   if (!s || !q || !qd || !jac) return -1;
@@ -775,23 +794,80 @@ int tds_b200_step_jacobian_device(tds_b200_sim* s, int mode, int use_pd, const f
   io.q_in = q; io.qd_in = qd; io.tau_in = tau_or_action;
   io.jac = jac; io.jac_n_in = dims[1];
   io.n = s->n; io.n_stride = s->ns;
-  const size_t warps = (size_t)(s->n + 31) / 32;
-  const size_t per_dir = warps * (size_t)s->dm_ad.x_total * 32 * 4;
-  const size_t cap = (size_t)2 << 30;                       // scratch bound: directions are processed in chunks
-  int chunk = (int)(cap / per_dir);
-  if (chunk < 1) chunk = 1;
-  if (chunk > dims[1]) chunk = dims[1];
-  if (per_dir * chunk > s->jac_scratch_bytes) {
-    if (s->jac_scratch) cudaFree(s->jac_scratch);
-    s->jac_scratch = nullptr; s->jac_scratch_bytes = 0;
-    CUDA_TRY(cudaMalloc((void**)&s->jac_scratch, per_dir * chunk));
-    s->jac_scratch_bytes = per_dir * chunk;
-  }
+  DualIO none;
+  memset(&none, 0, sizeof(none));
+  int chunk;
+  int rc = ensure_dual_scratch(s, dims[1], &chunk);
+  if (rc) return rc;
   for (int d0 = 0; d0 < dims[1]; d0 += chunk) {
     io.jac_dir0 = d0;
     const int nd = dims[1] - d0 < chunk ? dims[1] - d0 : chunk;
-    int rc = tds_launch_stepw_jacobian(&s->dm_ad, &s->P, &s->E, &io, mode, use_pd, nd, s->jac_scratch, (cudaStream_t)stream);
+    rc = tds_launch_stepw_dual(&s->dm_ad, &s->P, &s->E, &io, &none, mode, use_pd, nd, s->jac_scratch, (cudaStream_t)stream);
     if (rc) { set_err(std::string("jacobian launch: ") + cudaGetErrorString((cudaError_t)rc)); return rc; }
+  }
+  return 0;
+}
+
+// ---- Jacobian-vector and vector-Jacobian products of one step (same instance, same rows and columns as the dense Jacobian,
+// without the PD-gain columns).  Blocks: q [n_q], qd [n_qd], tau [n_tau] or action [n_act]; every array fp64 [dim][n_stride].
+static int dual_check(tds_b200_sim* s, int mode, int use_pd, const float* q, const float* qd, const float* tau_or_action,
+                      const char* what) {
+  if (!s || !q || !qd || mode < 0 || mode > 3) { set_err(std::string(what) + ": bad argument"); return -1; }
+  if (mode == 3) { set_err(std::string(what) + ": modes FD, NOCONTACT, FULL"); return -2; }
+  if (use_pd && s->E.n_act == 0) { set_err("use_pd without tds_b200_set_env"); return -3; }
+  if (use_pd && !tau_or_action) { set_err(std::string(what) + ": use_pd needs the actions"); return -1; }
+  return 0;
+}
+
+int tds_b200_step_jvp_device(tds_b200_sim* s, int mode, int use_pd, const float* q, const float* qd, const float* tau_or_action,
+                             const double* t_q, const double* t_qd, const double* t_tau, double* t_out, void* stream) {
+  int rc = dual_check(s, mode, use_pd, q, qd, tau_or_action, "step_jvp");
+  if (rc) return rc;
+  if (!t_out || (t_tau && !tau_or_action)) { set_err("step_jvp: bad argument"); return -1; }
+  StepIO io;
+  memset(&io, 0, sizeof(io));
+  io.q_in = q; io.qd_in = qd; io.tau_in = tau_or_action;
+  io.n = s->n; io.n_stride = s->ns;
+  DualIO dio;
+  memset(&dio, 0, sizeof(dio));
+  dio.jvp_tan[0] = t_q; dio.jvp_tan[1] = t_qd; dio.jvp_tan[2] = t_tau; dio.jvp_out = t_out;
+  int chunk;
+  if ((rc = ensure_dual_scratch(s, 1, &chunk))) return rc;
+  rc = tds_launch_stepw_dual(&s->dm_ad, &s->P, &s->E, &io, &dio, mode, use_pd, 1, s->jac_scratch, (cudaStream_t)stream);
+  if (rc) { set_err(std::string("jvp launch: ") + cudaGetErrorString((cudaError_t)rc)); return rc; }
+  return 0;
+}
+
+int tds_b200_step_vjp_device(tds_b200_sim* s, int mode, int use_pd, const float* q, const float* qd, const float* tau_or_action,
+                             const double* g_out, double* g_q, double* g_qd, double* g_tau, void* stream) {
+  int rc = dual_check(s, mode, use_pd, q, qd, tau_or_action, "step_vjp");
+  if (rc) return rc;
+  if (!g_out || (g_tau && !tau_or_action)) { set_err("step_vjp: bad argument"); return -1; }
+  const DevModel& M = s->dm[0];
+  const int n_in = use_pd ? s->E.n_act : s->n_tau;
+  const int first[3] = {0, M.n_q, M.n_q + M.n_qd}, count[3] = {M.n_q, M.n_qd, n_in};
+  double* const grad[3] = {g_q, g_qd, g_tau};
+  int dirs = 0;   // only the requested blocks are launched
+  for (int b = 0; b < 3; ++b) if (grad[b] && count[b] > dirs) dirs = count[b];
+  if (dirs == 0) return 0;
+  StepIO io;
+  memset(&io, 0, sizeof(io));
+  io.q_in = q; io.qd_in = qd; io.tau_in = tau_or_action;
+  io.n = s->n; io.n_stride = s->ns;
+  DualIO dio;
+  memset(&dio, 0, sizeof(dio));
+  dio.vjp_cot = g_out;
+  for (int b = 0; b < 3; ++b) dio.vjp_out[b] = grad[b];
+  int chunk;
+  if ((rc = ensure_dual_scratch(s, dirs, &chunk))) return rc;
+  for (int b = 0; b < 3; ++b) {
+    if (!grad[b]) continue;
+    for (int d0 = 0; d0 < count[b]; d0 += chunk) {
+      io.jac_dir0 = first[b] + d0;
+      const int nd = count[b] - d0 < chunk ? count[b] - d0 : chunk;
+      rc = tds_launch_stepw_dual(&s->dm_ad, &s->P, &s->E, &io, &dio, mode, use_pd, nd, s->jac_scratch, (cudaStream_t)stream);
+      if (rc) { set_err(std::string("vjp launch: ") + cudaGetErrorString((cudaError_t)rc)); return rc; }
+    }
   }
   return 0;
 }

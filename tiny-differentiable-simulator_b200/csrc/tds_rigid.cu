@@ -15,6 +15,7 @@
 
 #include "tds_math.cuh"
 #include "tds_dual.cuh"
+#include "tds_types.h"
 #include "tds_b200_model.h"
 
 #define TDS_RIGID_MAX_BODIES 16
@@ -100,13 +101,23 @@ TDS_D void plane_sphere(const V3<T>& pn, T pc, const V3<T>& c, T r, Contact<T>* 
 template <typename T, typename TS>
 __global__ void __launch_bounds__(128) tds_rigid_step_kernel(const __grid_constant__ RigidWorld W, const TS* s_in,
                                                              TS* s_out, const TS* __restrict__ force, int steps,
-                                                             int n, int ns, double* __restrict__ jac, int jac_dir0) {
+                                                             int n, int ns, double* __restrict__ jac, int jac_dir0,
+                                                             const DualIO dio = DualIO()) {
   const int e = blockIdx.x * blockDim.x + threadIdx.x;
   if (e >= n) return;
   constexpr bool AD = is_dual<T>::value;
   const int dir = AD ? (int)blockIdx.y + jac_dir0 : -1;      // differentiable instance: input direction of this lane
   const int nb = W.n_bodies;
-  auto seed = [&](T x, int idx) -> T { if constexpr (AD) { if (idx == dir) x.d = 1.0; } return x; };
+  // derivative part of input idx (blocks state 13 nb | force 3 nb): the caller's tangent (JVP), else d input_idx / d direction
+  auto seed = [&](T x, int idx) -> T {
+    if constexpr (AD) {
+      if (dio.jvp_out) {
+        const int blk = idx < 13 * nb ? 0 : 1, r = blk ? idx - 13 * nb : idx;
+        x.d = dio.jvp_tan[blk] ? dio.jvp_tan[blk][(size_t)r * ns + e] : 0.0;
+      } else if (idx == dir) x.d = 1.0;
+    }
+    return x;
+  };
   V3<T> pos[TDS_RIGID_MAX_BODIES], lin[TDS_RIGID_MAX_BODIES], ang[TDS_RIGID_MAX_BODIES];
   T qx[TDS_RIGID_MAX_BODIES], qy[TDS_RIGID_MAX_BODIES], qz[TDS_RIGID_MAX_BODIES], qw[TDS_RIGID_MAX_BODIES];
   // input directions: the 13 * n_bodies state entries, then the 3 * n_bodies force entries
@@ -218,15 +229,25 @@ __global__ void __launch_bounds__(128) tds_rigid_step_kernel(const __grid_consta
       qx[b] = x * inv; qy[b] = y * inv; qz[b] = z * inv; qw[b] = ww * inv;
     }
   }
+  double vjp_acc = 0.0;   // VJP: sum_r cot_r * d out_r / d direction
   for (int b = 0; b < nb; ++b) {
     const T out[13] = {pos[b].x, pos[b].y, pos[b].z, qx[b], qy[b], qz[b], qw[b], lin[b].x, lin[b].y, lin[b].z, ang[b].x, ang[b].y, ang[b].z};
     for (int k = 0; k < 13; ++k) {
       if constexpr (AD) {
-        if (jac) jac[((size_t)(b * 13 + k) * (16 * nb) + dir) * ns + e] = out[k].d;     // [row][column][world]
-        if (blockIdx.y == 0 && s_out) s_out[(size_t)(b * 13 + k) * ns + e] = (TS)val_of(out[k]);
+        const size_t r = (size_t)(b * 13 + k);
+        if (jac) jac[(r * (16 * nb) + dir) * ns + e] = out[k].d;     // [row][column][world]
+        if (dio.jvp_out) dio.jvp_out[r * ns + e] = out[k].d;
+        if (dio.vjp_cot) vjp_acc += dio.vjp_cot[r * ns + e] * out[k].d;
+        if (blockIdx.y == 0 && s_out) s_out[r * ns + e] = (TS)val_of(out[k]);
       } else {
         s_out[(size_t)(b * 13 + k) * ns + e] = (TS)out[k];
       }
+    }
+  }
+  if constexpr (AD) {
+    if (dio.vjp_cot) {
+      const int blk = dir < 13 * nb ? 0 : 1, r = blk ? dir - 13 * nb : dir;
+      if (dio.vjp_out[blk]) dio.vjp_out[blk][(size_t)r * ns + e] = vjp_acc;
     }
   }
 }
@@ -352,6 +373,54 @@ int tds_b200_rigid_jacobian_host(tds_b200_rigid* h, const double* state, const d
   for (int e = 0; e < n; ++e) {
     for (int k = 0; k < rows * cols; ++k) jac[(size_t)e * rows * cols + k] = t[(size_t)k * ns + e];
     if (state_out) for (int k = 0; k < rows; ++k) state_out[(size_t)e * rows + k] = so[(size_t)k * ns + e];
+  }
+  return 0;
+}
+
+// Products with d state_out / d (state | force) of `steps` steps, on device arrays in the layout of tds_b200_rigid_step_device; one
+// lane carries its derivative through all the steps.  A null force is zero force (a requested force block then differentiates at 0).
+static const double* rigid_force_or_zero(tds_b200_rigid* h, const double* force, bool needed, cudaStream_t sm) {
+  if (force || !needed) return force;
+  if (cudaMemsetAsync(h->force, 0, sizeof(double) * 3 * h->W.n_bodies * h->ns, sm) != cudaSuccess) return nullptr;
+  return h->force;
+}
+
+int tds_b200_rigid_jvp_device(tds_b200_rigid* h, const double* state, const double* force, int steps, const double* t_state,
+                              const double* t_force, double* t_out, void* stream) {
+  if (!h || !state || !t_out || steps < 0) return rigid_fail("rigid_jvp_device: bad argument", -1);
+  cudaStream_t sm = stream ? (cudaStream_t)stream : h->stream;
+  force = rigid_force_or_zero(h, force, t_force != nullptr, sm);
+  if (t_force && !force) return rigid_fail("rigid_jvp_device: zeroing the force failed", -1);
+  DualIO dio;
+  memset(&dio, 0, sizeof(dio));
+  dio.jvp_tan[0] = t_state; dio.jvp_tan[1] = t_force; dio.jvp_out = t_out;
+  const int T = 128;
+  tdsrb::tds_rigid_step_kernel<tds::Dual<double>, double><<<(h->n + T - 1) / T, T, 0, sm>>>(h->W, state, nullptr, force, steps, h->n, h->ns,
+                                                                                         nullptr, 0, dio);
+  RB_TRY(cudaGetLastError());
+  return 0;
+}
+
+int tds_b200_rigid_vjp_device(tds_b200_rigid* h, const double* state, const double* force, int steps, const double* g_out,
+                              double* g_state, double* g_force, void* stream) {
+  if (!h || !state || !g_out || steps < 0) return rigid_fail("rigid_vjp_device: bad argument", -1);
+  cudaStream_t sm = stream ? (cudaStream_t)stream : h->stream;
+  force = rigid_force_or_zero(h, force, g_force != nullptr, sm);
+  if (g_force && !force) return rigid_fail("rigid_vjp_device: zeroing the force failed", -1);
+  DualIO dio;
+  memset(&dio, 0, sizeof(dio));
+  dio.vjp_cot = g_out; dio.vjp_out[0] = g_state; dio.vjp_out[1] = g_force;
+  const int T = 128, nb = h->W.n_bodies;
+  // only the requested blocks are launched: directions [0, 13 nb) of the state, [13 nb, 16 nb) of the force
+  if (g_state) {
+    tdsrb::tds_rigid_step_kernel<tds::Dual<double>, double><<<dim3((h->n + T - 1) / T, 13 * nb), T, 0, sm>>>(
+        h->W, state, nullptr, force, steps, h->n, h->ns, nullptr, 0, dio);
+    RB_TRY(cudaGetLastError());
+  }
+  if (g_force) {
+    tdsrb::tds_rigid_step_kernel<tds::Dual<double>, double><<<dim3((h->n + T - 1) / T, 3 * nb), T, 0, sm>>>(
+        h->W, state, nullptr, force, steps, h->n, h->ns, nullptr, 13 * nb, dio);
+    RB_TRY(cudaGetLastError());
   }
   return 0;
 }

@@ -39,7 +39,7 @@ template <typename RA, typename RC, typename RS, typename RQ, bool SMEM>
 __global__ void __launch_bounds__(128, 1)
 tds_stepw_kernel(const __grid_constant__ DevModel M, const __grid_constant__ SimParams P,
                  const __grid_constant__ EnvParams E, const StepIO io, const int mode, const int use_pd,
-                 char* __restrict__ gscratch) {
+                 char* __restrict__ gscratch, const DualIO dio = DualIO()) {
   extern __shared__ __align__(16) char smem_raw[];
   const int lane = threadIdx.x & 31;
   const int warp_in_blk = threadIdx.x >> 5;
@@ -51,7 +51,6 @@ tds_stepw_kernel(const __grid_constant__ DevModel M, const __grid_constant__ Sim
   Arena A;
   if (SMEM) { A.blk = smem_raw + (size_t)warp_in_blk * M.x_total * 32 * 4; A.stride = 32; A.col = lane; }
   else { A.blk = gscratch + ((size_t)blockIdx.y * ((size_t)gridDim.x * (blockDim.x >> 5)) + (size_t)(env >> 5)) * M.x_total * 32 * 4; A.stride = 32; A.col = lane; }  // per-warp block, same addressing as shared memory
-  auto seed = [&](RQ x, int idx) -> RQ { if constexpr (AD) { if (idx == dir) x.d = 1.0; } return x; };   // d input_idx / d direction
   const int ST = A.stride;
   const int ns = io.n_stride;
   const int n_links = M.n_links;
@@ -81,6 +80,37 @@ tds_stepw_kernel(const __grid_constant__ DevModel M, const __grid_constant__ Sim
   // ---- load state, PD torques (locomotion_contact_simulation.h:168-258) ---------------------------
   // input directions of the differentiable instance: q | qd | tau or action | kp, kd, max_force (with PD)
   const int in0 = M.n_q + n;
+  // input direction idx -> its block (0 q, 1 qd, 2 tau or action) and its row there; -1: a PD gain (dense Jacobian only)
+  auto blk_of = [&](int idx, int& row) -> int {
+    if (idx < M.n_q) { row = idx; return 0; }
+    if (idx < in0) { row = idx - M.n_q; return 1; }
+    row = idx - in0;
+    return row < (use_pd ? E.n_act : n - (M.floating ? 6 : 0)) ? 2 : -1;
+  };
+  // derivative part of input idx: the caller's tangent (JVP), else d input_idx / d direction (Jacobian column, VJP)
+  auto seed = [&](RQ x, int idx) -> RQ {
+    if constexpr (AD) {
+      if (dio.jvp_out) { int r; const int b = blk_of(idx, r); x.d = (b >= 0 && dio.jvp_tan[b]) ? dio.jvp_tan[b][(size_t)r * ns + e] : 0.0; }
+      else if (idx == dir) x.d = 1.0;
+    }
+    return x;
+  };
+  // dual instance: output row r (q' | qd', or qdd in MODE_FD) has derivative d in this lane
+  double vjp_acc = 0.0;   // VJP: sum_r cot_r * d out_r / d direction
+  auto emit_row = [&](int r, double d) {
+    if constexpr (AD) {
+      if (io.jac) io.jac[((size_t)r * io.jac_n_in + dir) * ns + e] = d;
+      if (dio.jvp_out) dio.jvp_out[(size_t)r * ns + e] = d;
+      if (dio.vjp_cot) vjp_acc += dio.vjp_cot[(size_t)r * ns + e] * d;
+    }
+  };
+  auto store_vjp = [&]() {
+    if constexpr (AD) {
+      if (!dio.vjp_cot) return;
+      int r; const int b = blk_of(dir, r);
+      if (b >= 0 && dio.vjp_out[b]) dio.vjp_out[b][(size_t)r * ns + e] = vjp_acc;
+    }
+  };
   for (int k = 0; k < M.n_q; ++k) qv[k * ST] = seed(RQ(io.q_in[(size_t)k * ns + e]), k);
   for (int k = 0; k < n; ++k) qdv[k * ST] = seed(RQ(io.qd_in[(size_t)k * ns + e]), M.n_q + k);
   for (int k = 0; k < n; ++k) tauv[k * ST] = RQ(0.f);
@@ -662,7 +692,7 @@ tds_stepw_kernel(const __grid_constant__ DevModel M, const __grid_constant__ Sim
         a.top = axpy(S.top, qdd, a.top);
         a.bot = axpy(S.bot, qdd, a.bot);
         if (mode == MODE_FD) {
-          if constexpr (AD) { if (live && io.jac) io.jac[((size_t)(d0 + j) * io.jac_n_in + dir) * ns + e] = qdd.d; }
+          if constexpr (AD) { if (live) emit_row(d0 + j, qdd.d); }
           else if (live && io.qdd_out) io.qdd_out[(size_t)(d0 + j) * ns + e] = (float)val_of(qdd);
         } else if (!world_step) qdv[(d0 + j) * ST] = RQ(RA(qdv[(d0 + j) * ST]) + qdd * dtA);
       }
@@ -677,7 +707,7 @@ tds_stepw_kernel(const __grid_constant__ DevModel M, const __grid_constant__ Sim
       a.bot = axpy(S.bot, qdd, a.bot);
       const int qdi = M.qd_idx[i];
       if (mode == MODE_FD) {
-        if constexpr (AD) { if (live && io.jac) io.jac[((size_t)qdi * io.jac_n_in + dir) * ns + e] = qdd.d; }
+        if constexpr (AD) { if (live) emit_row(qdi, qdd.d); }
         else if (live && io.qdd_out) io.qdd_out[(size_t)qdi * ns + e] = (float)val_of(qdd);
       } else if (!world_step) qdv[qdi * ST] = RQ(RA(qdv[qdi * ST]) + qdd * dtA);
     }
@@ -690,13 +720,16 @@ tds_stepw_kernel(const __grid_constant__ DevModel M, const __grid_constant__ Sim
 #pragma unroll
     for (int k = 0; k < 6; ++k) {
       if (mode == MODE_FD) {
-        if constexpr (AD) { if (live && io.jac) io.jac[((size_t)k * io.jac_n_in + dir) * ns + e] = qb[k].d; }
+        if constexpr (AD) { if (live) emit_row(k, qb[k].d); }
         else if (live && io.qdd_out) io.qdd_out[(size_t)k * ns + e] = (float)val_of(qb[k]);
       } else if (!world_step) qdv[k * ST] = RQ(RC(qdv[k * ST]) + qb[k] * RC(P.dt));
     }
   }
   TDSW_PHASE();  // 4
-  if (mode == MODE_FD) return;
+  if (mode == MODE_FD) {
+    if constexpr (AD) { if (live) store_vjp(); }
+    return;
+  }
 
   // ---- contact solve -------------------------------------------------------------------------------------------
   __syncwarp();   // the Y rows below reuse the per-link records with another lane interleave
@@ -944,10 +977,11 @@ tds_stepw_kernel(const __grid_constant__ DevModel M, const __grid_constant__ Sim
   }
 
   // ---- reward / done / auto-reset, write back ------------------------------------------------------------------------
-  if constexpr (AD) {   // the Jacobian column of this lane's direction: rows q' | qd'
-    if (live && io.jac) {
-      for (int k = 0; k < M.n_q; ++k) io.jac[((size_t)k * io.jac_n_in + dir) * ns + e] = qv[k * ST].d;
-      for (int k = 0; k < n; ++k) io.jac[((size_t)(M.n_q + k) * io.jac_n_in + dir) * ns + e] = qdv[k * ST].d;
+  if constexpr (AD) {   // the Jacobian column of this lane's direction / the output tangents / the VJP entry: rows q' | qd'
+    if (live) {
+      for (int k = 0; k < M.n_q; ++k) emit_row(k, qv[k * ST].d);
+      for (int k = 0; k < n; ++k) emit_row(M.n_q + k, qdv[k * ST].d);
+      store_vjp();
     }
     return;
   }
@@ -998,7 +1032,7 @@ extern "C" int tds_launch_stepw(const DevModel* M, const SimParams* P, const Env
       if (err == cudaSuccess) smem_set = smem;                                                          \
     }                                                                                                   \
     if (err == cudaSuccess) {                                                                           \
-      k<<<blocks, threads, smem, stream>>>(*M, *P, *E, *io, mode, use_pd, gscratch);                    \
+      k<<<blocks, threads, smem, stream>>>(*M, *P, *E, *io, mode, use_pd, gscratch, DualIO());          \
       err = cudaGetLastError();                                                                         \
     }                                                                                                   \
   } while (0)
@@ -1009,15 +1043,16 @@ extern "C" int tds_launch_stepw(const DevModel* M, const SimParams* P, const Env
   return (int)err;
 }
 
-// Differentiable step: the same kernel on forward-mode dual numbers (fp64), one lane per (environment, input direction).
-// M must carry the 16-byte layout (tds_build_layout_w(..., 16, 16, 16, -1, 16)); gscratch: n_dirs * ceil(n / 32) blocks of
-// x_total * 128 bytes; directions [io->jac_dir0, io->jac_dir0 + n_dirs) are computed by this launch.
-extern "C" int tds_launch_stepw_jacobian(const DevModel* M, const SimParams* P, const EnvParams* E, const StepIO* io, int mode,
-                                         int use_pd, int n_dirs, char* gscratch, cudaStream_t stream) {
+// Differentiable step: the same kernel on forward-mode dual numbers (fp64).  M must carry the 16-byte layout
+// (tds_build_layout_w(..., 16, 16, 16, -1, 16)); gscratch: n_dirs * ceil(n / 32) blocks of x_total * 128 bytes.
+// Dense Jacobian (io->jac set) or VJP (dio->vjp_cot set): one lane per (environment, input direction) for directions
+// [io->jac_dir0, io->jac_dir0 + n_dirs).  JVP (dio->jvp_out set): one lane per environment, n_dirs = 1.
+extern "C" int tds_launch_stepw_dual(const DevModel* M, const SimParams* P, const EnvParams* E, const StepIO* io, const DualIO* dio,
+                                     int mode, int use_pd, int n_dirs, char* gscratch, cudaStream_t stream) {
   using namespace tdsw;
   typedef tds::Dual<double> D;
   const dim3 grid((io->n + 31) / 32, n_dirs);
-  tds_stepw_kernel<D, D, D, D, false><<<grid, 32, 0, stream>>>(*M, *P, *E, *io, mode, use_pd, gscratch);
+  tds_stepw_kernel<D, D, D, D, false><<<grid, 32, 0, stream>>>(*M, *P, *E, *io, mode, use_pd, gscratch, *dio);
   return (int)cudaGetLastError();
 }
 #endif  // TDS_STEPW_KERNEL_ONLY

@@ -140,3 +140,14 @@ struct StepIO {
   double* jac; int jac_n_in; int jac_dir0;
   int n; int n_stride;
 };
+
+// Products with the step's Jacobian, computed by the dual-number instances instead of (or besides) the dense Jacobian.
+// A trailing kernel parameter of its own, not part of StepIO: the float / double instances keep their parameter layout.
+// Input blocks: q | qd | tau or action (tds_stepw.cu), state | force (tds_rigid.cu); output rows as the dense Jacobian's.
+// Every array is fp64 [dim][n_stride].
+struct DualIO {
+  const double* jvp_tan[3];   // JVP (one lane per environment): tangent of each input block, null = zero
+  double* jvp_out;            // JVP: tangent of the output rows
+  const double* vjp_cot;      // VJP (one lane per environment and input direction): cotangent of the output rows
+  double* vjp_out[3];         // VJP: gradient of each input block; the lane of direction d writes sum_r cot_r * d out_r / d in_d
+};

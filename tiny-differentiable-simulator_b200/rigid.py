@@ -26,6 +26,12 @@ def plane(normal=(0.0, 0.0, 1.0), constant=0.0):
     return [0.0, PLANE, normal[0], normal[1], normal[2], constant]
 
 
+def _stream_arg(stream):
+    """None: the world's own stream.  A torch stream: that stream; torch's default stream (handle 0) is passed as
+    cudaStreamLegacy (1), since a null handle means the world's own stream to the tds_b200_rigid_*_device calls."""
+    return None if stream is None else ctypes.c_void_p(stream.cuda_stream or 1)
+
+
 def identity_state(n_worlds, n_bodies):
     """[n_worlds][n_bodies][13]: everything zero, orientations the identity quaternion (x, y, z, w) = (0, 0, 0, 1)."""
     s = np.zeros((n_worlds, n_bodies, 13))
@@ -93,10 +99,24 @@ class RigidWorld:
         return out, jac
 
     def step_device(self, state_in, state_out, force=None, steps=1, stream=None):
-        """CUDA tensors, fp64: state [13 * n_bodies][n_stride], force [3 * n_bodies][n_stride] or None; in place allowed."""
+        """CUDA tensors, fp64: state [13 * n_bodies][n_stride], force [3 * n_bodies][n_stride] or None; in place allowed.
+        stream: a torch stream (torch's default stream included), or None for the world's own stream."""
         p = lambda t: ctypes.c_void_p(t.data_ptr()) if t is not None else None
-        self._check(self._L.tds_b200_rigid_step_device(self._h, p(state_in), p(state_out), p(force), int(steps),
-                                                       ctypes.c_void_p(stream.cuda_stream) if stream is not None else None), "rigid_step_device")
+        self._check(self._L.tds_b200_rigid_step_device(self._h, p(state_in), p(state_out), p(force), int(steps), _stream_arg(stream)),
+                    "rigid_step_device")
+
+    def jvp_device(self, state, force, steps, t_state, t_force, t_out, stream=None):
+        """Jacobian-vector product of `steps` steps with respect to (state | force), CUDA tensors fp64 in the layouts of step_device:
+        tangents t_state [13 * n_bodies][n_stride], t_force [3 * n_bodies][n_stride] or None (zero) -> t_out like state."""
+        p = lambda t: ctypes.c_void_p(t.data_ptr()) if t is not None else None
+        self._check(self._L.tds_b200_rigid_jvp_device(self._h, p(state), p(force), int(steps), p(t_state), p(t_force), p(t_out),
+                                                      _stream_arg(stream)), "rigid_jvp_device")
+
+    def vjp_device(self, state, force, steps, g_out, g_state=None, g_force=None, stream=None):
+        """Vector-Jacobian product of `steps` steps: g_out (cotangent of the new state) -> g_state, g_force (None: not computed)."""
+        p = lambda t: ctypes.c_void_p(t.data_ptr()) if t is not None else None
+        self._check(self._L.tds_b200_rigid_vjp_device(self._h, p(state), p(force), int(steps), p(g_out), p(g_state), p(g_force),
+                                                      _stream_arg(stream)), "rigid_vjp_device")
 
     @property
     def n_stride(self):

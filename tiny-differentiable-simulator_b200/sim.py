@@ -40,6 +40,7 @@ class BatchSim:
         (self.n_envs, self.n_stride, self.n_q, self.n_qd, self.n_tau, self.n_links,
          self.n_contact_points, self.n_act) = list(dims)
         self.device = device
+        self.auto_reset = False
         self.set_params(dt, gravity, friction, restitution, erp, cfm, pgs_iterations, keep_all_points)
         self.set_precision(precision)
 
@@ -83,6 +84,7 @@ class BatchSim:
         if rq is not None:
             assert rq.size == self.n_q
         self._check(self._L.tds_b200_set_auto_reset(self._h, int(enable), _dp(rq)), "set_auto_reset")
+        self.auto_reset = bool(enable)
 
     def kernel_name(self):
         """Step kernel launched by the last step call (after the library's selection / fallbacks)."""
@@ -157,6 +159,24 @@ class BatchSim:
         jac = np.zeros((self.n_envs, dims[0], dims[1]))
         self._check(self._L.tds_b200_step_jacobian_host(self._h, mode, int(use_pd), _dp(q), _dp(qd), _dp(t), _dp(jac)), "step_jacobian_host")
         return jac
+
+    def step_jvp_device(self, mode, q, qd, tau_or_action, t_q, t_qd, t_tau, t_out, use_pd=False, stream=None):
+        """Jacobian-vector product of one step on the device, without the dense Jacobian: q, qd, tau_or_action as for step_device
+        (float32 [dim, n_stride]); tangents t_q, t_qd, t_tau float64 [dim, n_stride] or None (zero); t_out float64
+        [rows, n_stride] receives the tangent of q' | qd' (of qdd for MODE_FD).  Columns e >= n_envs are not written."""
+        import torch
+        st = ctypes.c_void_p(stream.cuda_stream if stream is not None else torch.cuda.current_stream().cuda_stream)
+        self._check(self._L.tds_b200_step_jvp_device(self._h, mode, int(use_pd), _ptr(q), _ptr(qd), _ptr(tau_or_action), _ptr(t_q),
+                                                     _ptr(t_qd), _ptr(t_tau), _ptr(t_out), st), "step_jvp_device")
+
+    def step_vjp_device(self, mode, q, qd, tau_or_action, g_out, g_q=None, g_qd=None, g_tau=None, use_pd=False, stream=None):
+        """Vector-Jacobian product of one step on the device: g_out float64 [rows, n_stride] is the cotangent of q' | qd' (of qdd
+        for MODE_FD); g_q, g_qd, g_tau float64 [dim, n_stride] receive the gradient of each input block, or None: that block is
+        not computed (its dual lanes are not launched)."""
+        import torch
+        st = ctypes.c_void_p(stream.cuda_stream if stream is not None else torch.cuda.current_stream().cuda_stream)
+        self._check(self._L.tds_b200_step_vjp_device(self._h, mode, int(use_pd), _ptr(q), _ptr(qd), _ptr(tau_or_action), _ptr(g_out),
+                                                     _ptr(g_q), _ptr(g_qd), _ptr(g_tau), st), "step_vjp_device")
 
     def integrate_host(self, q, qd, qdd, update_q=True):
         """integrate_euler (update_q) / integrate_euler_qdd of one state vector per environment, on the device
